@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA engine
     python bench.py --impl reference [--gpus N] ...                # CPU arm (oracle port, all host threads)
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N   # one rank per GPU
+    python bench.py ... --dump-outputs DIR                          # + what the last timed step computed, DIR/<name>.npy
 
 One "step" = one Monte Carlo iteration of the hot path (`montecarlo_transport_with_vpackets`,
 tardis/transport/montecarlo/modes/montecarlo_transport.py:239) over one batch of synthetic packets, INCLUDING what
@@ -358,9 +359,32 @@ class Rig:
         return {k: t.numpy() for k, t in self.out_pins["t"].items()}
 
 
-def measure(rig: Rig, spec: dict, model, steps: int, warmup: int, e2e_steps: int, with_clocks: bool, device_source: bool):
+DUMP_SAMPLE = 1 << 20  # entries kept per dumped array: four sampled arrays of 8 MB each keep a dump near 32 MB
+DUMP_SEED = 20240917
+
+
+def dump_outputs(res: dict, out_dir: str):
+    """What the caller of the timed path receives after its last step (`res`: the engine's download of it), as
+    <out_dir>/<name>.npy in float64: the per-packet outputs, the estimators, the fused spectra and luminosity sums, and the work
+    counters.  An array larger than DUMP_SAMPLE entries is reduced to the same seeded, sorted sample of its flattened entries on
+    every run, so two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    res = dict(res)
+    counters = res.pop("counters")
+    res["counters"] = np.array([counters[k] for k in sorted(counters)], dtype=np.float64)  # sorted counter names
+    for name, a in res.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.size > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(a.size, DUMP_SAMPLE, replace=False))
+            a = a.ravel()[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def measure(rig: Rig, spec: dict, model, steps: int, warmup: int, e2e_steps: int, with_clocks: bool, device_source: bool,
+            dump_dir: str | None = None):
     """One workload on this rank's engine: resident steps, end-to-end steps, cross-rank check.  Returns the leg's dict
-    (rank 0 adds roofline / cpu_baseline / parity afterwards)."""
+    (rank 0 adds roofline / cpu_baseline / parity afterwards).  With `dump_dir`, rank 0 writes what the last timed step computed
+    there (dump_outputs) before anything else runs on the engine."""
     from tardis_b200 import parallel
 
     torch, dist, eng, world, args = rig.torch, rig.dist, rig.eng, rig.world, rig.args
@@ -403,6 +427,8 @@ def measure(rig: Rig, spec: dict, model, steps: int, warmup: int, e2e_steps: int
     launches = eng.kernel_launches() - launches0
     counters = eng.counters()
     value = n_total * steps / elapsed
+    if dump_dir is not None and rig.rank == 0:
+        dump_outputs(eng.download(), dump_dir)
 
     # ---- cross-rank check of the collective (N > 1): sum over ranks of the local buffers == the all-reduced buffer ----
     cross = None
@@ -812,7 +838,14 @@ def main():
                          "(default: all when the headline is the default workload, none otherwise)")
     ap.add_argument("--leg-steps", type=int, default=3)
     ap.add_argument("--leg-scale", type=float, default=1.0, help="scale the legs' packet counts (quick runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the headline's last timed step computed to DIR/<name>.npy (float64; arrays above "
+                         f"{DUMP_SAMPLE} entries as a fixed seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200: the reference arm's sample size is calibrated from its timing")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -892,7 +925,8 @@ def main():
     rig.ensure_packets(n_max, model.r_inner[0])
     use_ds = not args.no_device_source
     e2e_steps = max(1, args.steps)
-    headline = measure(rig, head, model, args.steps, args.warmup, e2e_steps, with_clocks=True, device_source=use_ds)
+    headline = measure(rig, head, model, args.steps, args.warmup, e2e_steps, with_clocks=True, device_source=use_ds,
+                       dump_dir=args.dump_outputs)
 
     if rank == 0:
         n = headline["_n"]

@@ -449,10 +449,75 @@ def generate_formal_integral(name):
     print(f"{name}: wrote {os.path.getsize(path)/1e3:.0f} kB; L_nu in [{keep['luminosity_densities'].min():.3e}, {keep['luminosity_densities'].max():.3e}]")
 
 
+# The reference's public surface the host mirrors keep (tests/test_interface_mirror.py, tests/test_packet_source.py): positional
+# parameter names of each mirrored function, per source file (paths relative to tardis/transport/montecarlo/modes, as the tests
+# name them), parsed with ast and never imported.
+INTERFACE_SIGNATURES = {
+    "montecarlo_transport.py": ["montecarlo_transport_with_vpackets"],
+    "iip/montecarlo_transport.py": ["montecarlo_transport"],
+    "classic/solver.py": ["MCTransportSolverClassic.__init__", "MCTransportSolverClassic.from_config",
+                          "MCTransportSolverClassic.initialize_transport_state", "MCTransportSolverClassic.run"],
+    "iip/solver.py": ["MCTransportSolverIIP.__init__", "MCTransportSolverIIP.from_config", "MCTransportSolverIIP.initialize_transport_state",
+                      "MCTransportSolverIIP.run"],
+    "../estimators/mc_rad_field_solver.py": ["MCRadiationFieldPropertiesSolver.__init__", "MCRadiationFieldPropertiesSolver.solve"],
+    "../../../spectrum/formal_integral/source_function.py": ["SourceFunctionSolver.__init__", "SourceFunctionSolver.solve"],
+    "../../../spectrum/formal_integral/formal_integral_solver.py": ["FormalIntegralSolver.__init__", "FormalIntegralSolver.solve"],
+    "../../../spectrum/formal_integral/base.py": ["check_formal_integral_requirements"],
+    "../../../spectrum/base.py": ["SpectrumSolver.__init__", "SpectrumSolver.setup_optional_spectra", "SpectrumSolver.solve",
+                                  "SpectrumSolver.from_config"],
+    "../../../spectrum/spectrum.py": ["TARDISSpectrum.__init__"],
+}
+
+
+def generate_reference_interface():
+    """tests/golden/reference_interface.json: the mirrored signatures (INTERFACE_SIGNATURES), SpectrumSolver's properties and
+    hdf_properties, and the public methods of BasePacketSource / BlackBodySimpleSource."""
+    import ast
+    import json
+
+    from oracle.reference_loader import REF
+
+    modes = os.path.join(REF, "tardis", "transport", "montecarlo", "modes")
+
+    def parse(rel):
+        with open(os.path.normpath(os.path.join(modes, rel))) as f:
+            return ast.parse(f.read())
+
+    signatures = {}
+    for rel, names in INTERFACE_SIGNATURES.items():
+        found = {}
+        for node in parse(rel).body:
+            if isinstance(node, ast.FunctionDef):
+                found[node.name] = [a.arg for a in node.args.args]
+            elif isinstance(node, ast.ClassDef):
+                for m in node.body:
+                    if isinstance(m, ast.FunctionDef):
+                        found[f"{node.name}.{m.name}"] = [a.arg for a in m.args.args if a.arg not in ("self", "cls")]
+        signatures[rel] = {n: found[n] for n in names}
+    cls = next(n for n in parse("../../../spectrum/base.py").body if isinstance(n, ast.ClassDef) and n.name == "SpectrumSolver")
+    props = [m.name for m in cls.body if isinstance(m, ast.FunctionDef) and any(getattr(d, "id", None) == "property" for d in m.decorator_list)]
+    hdf = next(ast.literal_eval(m.value) for m in cls.body if isinstance(m, ast.Assign) and m.targets[0].id == "hdf_properties")
+    packet_source = set()
+    for f in ("base.py", "black_body.py"):
+        for node in parse(os.path.join("..", "packet_source", f)).body:
+            if isinstance(node, ast.ClassDef) and node.name in ("BasePacketSource", "BlackBodySimpleSource"):
+                packet_source |= {m.name for m in node.body if isinstance(m, ast.FunctionDef) and not m.name.startswith("_")}
+    out = {"signatures": signatures, "spectrum_solver": {"properties": props, "hdf_properties": hdf},
+           "packet_source_public_methods": sorted(packet_source)}
+    path = os.path.join(HERE, "reference_interface.json")
+    with open(path, "w") as f:
+        json.dump(out, f, indent=1, sort_keys=True)
+        f.write("\n")
+    print(f"reference_interface: wrote {os.path.getsize(path)} bytes")
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--case", default=None)
     args = ap.parse_args()
+    if args.case == "reference_interface":
+        generate_reference_interface()
+        return
     if args.case in PACKET_SOURCE_CASES:
         generate_packet_source(args.case)
         return
@@ -506,6 +571,7 @@ def main():
     subprocess.run([sys.executable, os.path.abspath(__file__), "--case", "source_function_bench_shape"], check=True)
     subprocess.run([sys.executable, os.path.abspath(__file__), "--case", "opacity_bench_shape"], check=True)
     subprocess.run([sys.executable, os.path.abspath(__file__), "--case", "radfield_bench_shape"], check=True)
+    generate_reference_interface()
 
 
 if __name__ == "__main__":

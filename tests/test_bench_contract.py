@@ -193,3 +193,61 @@ def test_tables_block_plumbing_with_a_stub_engine(monkeypatch):
     assert "error" not in sp, sp.get("error")
     assert sp["shells_checked"] == [0, 2, 4] and all(sp[k]["zero_pattern_equal"] and sp[k]["max_err_over_bar"] <= 1.0 for k in ("att_S_ul", "Jred_lu", "Jblue_lu"))
     assert out["source_function"]["sweeps"] == 24 and out["host_tables"]["ms"] >= 0 and out["device_tables"]["n_levels"] == 3000
+
+
+def test_dump_outputs_writes_float64_with_a_fixed_sample_of_large_arrays(tmp_path):
+    """bench.py --dump-outputs: every array of the result as <name>.npy in float64, counters as one array in sorted-name order, and
+    an array above DUMP_SAMPLE entries as the same sorted sample of its flat entries on every call."""
+    import numpy as np
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    n = 3 * bench.DUMP_SAMPLE
+    res = {"output_nus": np.arange(n, dtype=np.float64), "j": np.linspace(1.0, 2.0, 20), "j_blue": np.arange(n, dtype=np.float64).reshape(-1, 3),
+           "photo_ion_estimator_statistics": np.arange(12, dtype=np.int64).reshape(3, 4), "counters": {"n_line_steps": 7, "n_boundary_events": 5}}
+    for d in ("a", "b"):
+        bench.dump_outputs(res, str(tmp_path / d))
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["counters.npy", "j.npy", "j_blue.npy", "output_nus.npy", "photo_ion_estimator_statistics.npy"]
+    for name in names:
+        a, b = np.load(tmp_path / "a" / name), np.load(tmp_path / "b" / name)
+        assert a.dtype == np.float64 and np.array_equal(a, b), name
+    assert np.array_equal(np.load(tmp_path / "a" / "counters.npy"), [5.0, 7.0])
+    assert np.array_equal(np.load(tmp_path / "a" / "j.npy"), res["j"])
+    assert np.array_equal(np.load(tmp_path / "a" / "photo_ion_estimator_statistics.npy"), res["photo_ion_estimator_statistics"])
+    s = np.load(tmp_path / "a" / "output_nus.npy")  # the values are their own indices: a sorted sample without repeats
+    assert s.shape == (bench.DUMP_SAMPLE,) and np.all(np.diff(s) > 0) and s[-1] < n
+    assert np.array_equal(np.load(tmp_path / "a" / "j_blue.npy"), s)  # same size -> same flat positions
+
+
+def test_dump_outputs_is_refused_on_the_reference_arm(tmp_path):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path / "d")],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode != 0 and "--dump-outputs" in out.stderr and not (tmp_path / "d").exists()
+
+
+@pytest.mark.gpu
+def test_bench_dumps_identical_inputs_outputs_on_every_run(tmp_path):
+    """A small headline run twice with --dump-outputs: the JSON line reports the requested steps, the dump stays within 64 MB of
+    float64 arrays, and the same arguments give the same outputs (integer work exactly, floating-point sums to the last bits)."""
+    import numpy as np
+
+    args = ["--gpus", "1", "--steps", "2", "--warmup", "1", "--packets", "200000", "--lines", "20000", "--shells", "10", "--mu-tau", "-4.5",
+            "--legs", "none", "--no-cpu-baseline", "--no-tables", "--no-scan-reference", "--no-device-source"]
+    for d in ("a", "b"):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args, "--dump-outputs", str(tmp_path / d)],
+                             capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-3000:]
+        line = json.loads([ln for ln in out.stdout.splitlines() if ln.startswith("{")][-1])
+        assert line["steps"] == 2 and line["warmup"] == 1 and line["gpu_launches"] >= 7 * 2
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert {"output_nus.npy", "output_energies.npy", "j.npy", "nu_bar.npy", "j_blue.npy", "edotlu.npy", "counters.npy"} <= set(names)
+    assert sum(os.path.getsize(tmp_path / "a" / n) for n in names) <= 64 << 20
+    for name in names:
+        a, b = np.load(tmp_path / "a" / name), np.load(tmp_path / "b" / name)
+        assert a.dtype == np.float64 and a.shape == b.shape, name
+        np.testing.assert_allclose(a, b, rtol=1e-12, atol=0, err_msg=name)
+    assert np.array_equal(np.load(tmp_path / "a" / "counters.npy"), np.load(tmp_path / "b" / "counters.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "output_nus.npy"), np.load(tmp_path / "b" / "output_nus.npy"))
+    assert np.load(tmp_path / "a" / "output_nus.npy").shape == (200000,)

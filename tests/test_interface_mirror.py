@@ -1,8 +1,8 @@
 """The host mirror keeps the reference's call signatures for the hot path (SURVEY.md §8b): every positional parameter of
-the reference, same name, same order; ours may only append keyword extras.  The reference's sources are parsed (not
-imported), so this runs wherever /root/reference exists and is skipped elsewhere (the GPU box)."""
-import ast
+the reference, same name, same order; ours may only append keyword extras.  The reference's signatures were parsed from its
+sources (not imported) into tests/golden/reference_interface.json by tests/golden/make_golden.py --case reference_interface."""
 import inspect
+import json
 import os
 
 import pytest
@@ -12,21 +12,8 @@ from tardis_b200 import formal_integral as fim
 from tardis_b200 import source_function as sfm
 from tardis_b200 import spectrum as spm
 
-REF = "/root/reference/tardis/transport/montecarlo/modes"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
-
-
-def ref_signatures(path):
-    out = {}
-    tree = ast.parse(open(os.path.join(REF, path)).read())
-    for node in tree.body:
-        if isinstance(node, ast.FunctionDef):
-            out[node.name] = [a.arg for a in node.args.args]
-        elif isinstance(node, ast.ClassDef):
-            for m in node.body:
-                if isinstance(m, ast.FunctionDef):
-                    out[f"{node.name}.{m.name}"] = [a.arg for a in m.args.args if a.arg not in ("self", "cls")]
-    return out
+with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_interface.json")) as _f:
+    REF = json.load(_f)
 
 
 def ours(obj):
@@ -59,18 +46,15 @@ def ours(obj):
     ("../../../spectrum/spectrum.py", "TARDISSpectrum.__init__", spm.TARDISSpectrumB200.__init__),
 ])
 def test_mirror_keeps_reference_parameters(ref_file, ref_name, mirror):
-    ref = ref_signatures(ref_file)[ref_name]
+    ref = REF["signatures"][ref_file][ref_name]
     mine = ours(mirror)
     assert mine[:len(ref)] == ref, (ref_name, ref, mine)
 
 
 def test_spectrum_solver_mirror_has_the_reference_s_properties():
     """every property / attribute list of SpectrumSolver (spectrum/base.py:14-202) exists on the mirror under the same name"""
-    tree = ast.parse(open(os.path.join(REF, "../../../spectrum/base.py")).read())
-    cls = next(n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == "SpectrumSolver")
-    props = [m.name for m in cls.body if isinstance(m, ast.FunctionDef) and any(getattr(d, "id", None) == "property" for d in m.decorator_list)]
+    props = REF["spectrum_solver"]["properties"]
     assert len(props) >= 8
     for name in props:
         assert isinstance(getattr(spm.SpectrumSolverB200, name), property), name
-    hdf = next(ast.literal_eval(m.value) for m in cls.body if isinstance(m, ast.Assign) and m.targets[0].id == "hdf_properties")
-    assert spm.SpectrumSolverB200.hdf_properties == hdf and spm.SpectrumSolverB200.hdf_name == "spectrum"
+    assert spm.SpectrumSolverB200.hdf_properties == REF["spectrum_solver"]["hdf_properties"] and spm.SpectrumSolverB200.hdf_name == "spectrum"
